@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (N>1: launched by torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU/gloo path
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR  # + the last step's loss / parameters / gradients
 
 Workload (BASELINE.json configs[1]): torchvision resnet50 (random init, seed 0), synthetic
 224x224 images, per-GPU batch 64, bf16 autocast, SGD momentum, DDP with
@@ -61,7 +62,38 @@ def parse():
     ap.add_argument("--optimizer-in-backward", action="store_true",
                     help="apply the optimizer per DDP bucket right behind its allreduce (f-2; SGD / Adam / AdamW)")
     ap.add_argument("--cpu-batch", type=int, default=8)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss, parameters and gradients of the last step as DIR/*.npy "
+                         "(convolutions then use deterministic cuDNN algorithms, so that runs can be compared)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_SAMPLE = 1 << 22   # elements kept of a longer flat array: 16 MiB of float32, so at most 32 MiB in all
+
+
+def dump_outputs(out_dir, torch, model, loss):
+    """Write what a caller of the training step holds after the last timed step, so that two builds can be compared
+    output for output: the loss (float64) and every parameter and its synchronised gradient, concatenated flat in
+    ``model.parameters()`` order (float32).  A flat array longer than DUMP_SAMPLE elements is cut down to the same
+    seeded sample of positions in every run; gradients are written only when every parameter has one."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    params = list(model.parameters())
+    flat = {"params": torch.cat([p.detach().float().reshape(-1) for p in params])}
+    if all(p.grad is not None for p in params):
+        flat["grads"] = torch.cat([p.grad.detach().float().reshape(-1) for p in params])
+    n = flat["params"].numel()
+    idx = None
+    if n > DUMP_SAMPLE:
+        idx = torch.randint(0, n, (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+    for name, t in flat.items():
+        if idx is not None:
+            t = t[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([float(loss)], dtype=np.float64))
 
 
 def free_port():
@@ -412,7 +444,12 @@ def run_b200(args):
     os.environ.setdefault("PL_TORCH_DISTRIBUTED_BACKEND", "nccl")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
-    torch.backends.cudnn.benchmark = True
+    # cuDNN's autotuner picks convolution algorithms by timing them in each run, and some of them accumulate with
+    # atomics, so the same inputs give different outputs from run to run.  Outputs written for comparison come from
+    # deterministic algorithms instead; at the default ResNet-50 workload they are no slower (17.36 ms/step against
+    # 17.46 autotuned, one B200 at a 1000 W power limit, mean of two runs each).
+    torch.backends.cudnn.benchmark = not args.dump_outputs
+    torch.backends.cudnn.deterministic = bool(args.dump_outputs)
 
     import torchvision
     torch.manual_seed(0)
@@ -556,6 +593,9 @@ def run_b200(args):
     exch_ms, exch_timed, exch_launches = float(st.get("exch_ms", 0.0)), int(st.get("exch_timed", 0)), int(st.get("exch_launches", 0))
     last_algo = int(st.get("last_algo", 0))
     e2e_ms, last_loss = timed(args.steps, e2e=True)
+    if args.dump_outputs and rank == 0:
+        # right after the last timed step: the isolated runs below push random data through the same bucket slots
+        dump_outputs(args.dump_outputs, torch, model, last_loss)
 
     # The same buckets once more, ISOLATED (no backward running, ranks aligned by a barrier): what the
     # kernel does when it is not waiting for SMs or for a slower peer.  Through the same hook entry point.

@@ -1,37 +1,22 @@
-"""The plugin surface is the reference's, checked against the reference SOURCE by AST (it cannot be
-imported: ray / pytorch_lightning are absent).  Runs where /root/reference exists (the build
-container); skipped on the GPU box."""
-import ast
+"""The plugin surface is the reference's: ray_lightning's classes and module names, read from its source by AST
+(oracle/make_surface_golden.py, stored in tests/golden/reference_surface.json), against this package's."""
 import inspect
+import json
 import os
 
 import pytest
 
-REF = "/root/reference/ray_lightning"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources not present on this box")
+REF_SURFACE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_surface.json")
 
 
-def _cls(path, name):
-    tree = ast.parse(open(os.path.join(REF, path)).read())
-    for node in ast.walk(tree):
-        if isinstance(node, ast.ClassDef) and node.name == name:
-            return node
-    raise KeyError(name)
-
-
-def _methods(node):
-    return {n.name: n for n in node.body if isinstance(n, ast.FunctionDef)}
-
-
-def _sig(fn):
-    a = fn.args
-    names = [x.arg for x in a.args]
-    defaults = [None] * (len(names) - len(a.defaults)) + [ast.literal_eval(d) if isinstance(d, ast.Constant) else "<expr>" for d in a.defaults]
-    return list(zip(names, defaults)), (a.vararg.arg if a.vararg else None), (a.kwarg.arg if a.kwarg else None), \
-        [k.arg for k in a.kwonlyargs]
+@pytest.fixture(scope="module")
+def ref():
+    with open(REF_SURFACE) as f:
+        return json.load(f)
 
 
 def _mine(fn):
+    """fn's signature in the stored form: [[[name, default], ...], vararg, kwarg, [kwonly, ...]]."""
     sig = inspect.signature(fn)
     pos, var, kw, kwonly = [], None, None, []
     for p in sig.parameters.values():
@@ -42,60 +27,50 @@ def _mine(fn):
         elif p.kind == p.KEYWORD_ONLY:
             kwonly.append(p.name)
         else:
-            pos.append((p.name, None if p.default is p.empty else p.default))
-    return pos, var, kw, kwonly
+            pos.append([p.name, None if p.default is p.empty else p.default])
+    return [pos, var, kw, kwonly]
 
 
-def test_ray_strategy_surface():
+def test_ray_strategy_surface(ref):
     from ray_lightning_b200 import RayStrategy
-    ref = _cls("ray_ddp.py", "RayStrategy")
-    rm = _methods(ref)
-    assert _sig(rm["__init__"]) == _mine(RayStrategy.__init__)
-    for name, fn in rm.items():
+    rm = ref["RayStrategy"]
+    assert rm["__init__"] == _mine(RayStrategy.__init__)
+    for name, sig in rm.items():
         assert hasattr(RayStrategy, name), name
         if name != "__init__" and not isinstance(inspect.getattr_static(RayStrategy, name), property):
-            assert _sig(fn)[0] == _mine(getattr(RayStrategy, name))[0], name
+            assert sig[0] == _mine(getattr(RayStrategy, name))[0], name
     assert RayStrategy.strategy_name == "ddp_ray"
 
 
-def test_sharded_and_horovod_surface():
+def test_sharded_and_horovod_surface(ref):
     from ray_lightning_b200 import HorovodRayStrategy, RayShardedStrategy
     assert RayShardedStrategy.strategy_name == "ddp_sharded_ray"
-    ref = _cls("ray_horovod.py", "HorovodRayStrategy")
-    rm = _methods(ref)
-    assert _sig(rm["__init__"]) == _mine(HorovodRayStrategy.__init__)
+    rm = ref["HorovodRayStrategy"]
+    assert rm["__init__"] == _mine(HorovodRayStrategy.__init__)
     for name in rm:
         assert hasattr(HorovodRayStrategy, name), name
     assert HorovodRayStrategy.strategy_name == "horovod_ray"
 
 
-def test_launcher_and_executor_surface():
+def test_launcher_and_executor_surface(ref):
     from ray_lightning_b200.launchers import RayHorovodLauncher, RayLauncher
     from ray_lightning_b200.launchers.utils import _RayExecutorImpl, _RayOutput
-    rm = _methods(_cls("launchers/ray_launcher.py", "RayLauncher"))
-    for name, fn in rm.items():
+    for name, sig in ref["RayLauncher"].items():
         assert hasattr(RayLauncher, name), name
-        assert _sig(fn) == _mine(getattr(RayLauncher, name)), name
-    ex = _methods(_cls("launchers/utils.py", "RayExecutor"))
-    for name, fn in ex.items():
-        assert _sig(fn) == _mine(getattr(_RayExecutorImpl, name)), name
-    out = _cls("launchers/utils.py", "_RayOutput")
-    fields = [n.target.id for n in out.body if isinstance(n, ast.AnnAssign)]
-    assert list(_RayOutput._fields) == fields
-    hv = _methods(_cls("launchers/ray_horovod_launcher.py", "RayHorovodLauncher"))
-    assert _sig(hv["launch"]) == _mine(RayHorovodLauncher.launch)
+        assert sig == _mine(getattr(RayLauncher, name)), name
+    for name, sig in ref["RayExecutor"].items():
+        assert sig == _mine(getattr(_RayExecutorImpl, name)), name
+    assert list(_RayOutput._fields) == ref["_RayOutput_fields"]
+    assert ref["RayHorovodLauncher"]["launch"] == _mine(RayHorovodLauncher.launch)
 
 
-def test_module_level_names():
+def test_module_level_names(ref):
     import ray_lightning_b200 as pkg
     from ray_lightning_b200 import session, tune, util
-    tree = ast.parse(open(os.path.join(REF, "__init__.py")).read())
-    ref_all = next(ast.literal_eval(n.value) for n in tree.body if isinstance(n, ast.Assign) and n.targets[0].id == "__all__")
-    assert sorted(pkg.__all__) == sorted(ref_all)
-    for mod, path in ((session, "session.py"), (util, "util.py")):
-        t = ast.parse(open(os.path.join(REF, path)).read())
-        for n in t.body:
-            if isinstance(n, (ast.FunctionDef, ast.ClassDef)) and n.name != "DelayedGPUAccelerator":
-                assert hasattr(mod, n.name), (path, n.name)
+    assert sorted(pkg.__all__) == sorted(ref["__all__"])
+    for mod, key in ((session, "session_names"), (util, "util_names")):
+        for name in ref[key]:
+            if name != "DelayedGPUAccelerator":
+                assert hasattr(mod, name), (key, name)
     for name in ("TuneReportCallback", "TuneReportCheckpointCallback", "get_tune_resources", "is_session_enabled", "TUNE_INSTALLED"):
         assert hasattr(tune, name)
